@@ -50,13 +50,60 @@ def parse_args():
                     help="BASELINE.json config: 2 = headline (1080p JPEG -> 256x256 JPEG), 3 = 4K RGBA PNG -> 512x512 "
                          "WebP, 4 = 128-frame 720p GIF -> 256x256 animated WebP, 5 = mixed JPEG/PNG/WebP -> 256x256 JPEG")
     ap.add_argument("--distinct", type=int, default=0, help="configs 3-5: distinct files generated (replicated to the batch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(see dump_outputs): status, length and CRC-32 of every output, but the bytes of a seeded "
+                         "sample only, sized for outputs at full capacity (192 of 4096 for config 2, one animation "
+                         "for config 4); with more than one rank, each rank writes DIR/rank<r>/")
     ap.add_argument("--variant", default="default", choices=["default", "cv2", "optimized", "dri", "pcg64"],
                     help="config 2 corpus: default = this library's encoder (byte-identical to the reference's); cv2 = "
                          "OpenCV / libjpeg-turbo written files; optimized = per-image optimised Huffman tables (a DHT "
                          "per file); dri = restart interval of one MCU row; pcg64 = SURVEY 8(d)'s generator to the letter "
                          "(numpy PCG64(1000 + i) content made on the host CPUs, files written by libjpeg-turbo; ~0.7 s "
                          "per image and core, so use it with a smaller --batch).  Secondary, labelled lines.")
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm returns no outputs to the bench")
+    return args
+
+
+# ------------------------------------------------------------------------------ output dump
+
+DUMP_SAMPLE_BYTES = 48 << 20   # float32 budget of the sampled files: the whole dump stays under 64 MB
+
+
+def dump_sample(n, out_cap):
+    """Sorted indices of the items whose encoded files are dumped: a seeded draw that depends only on the item
+    count and the output capacity, never on the outputs, so two builds dump the same items."""
+    k = min(n, max(1, DUMP_SAMPLE_BYTES // (4 * out_cap)))
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def dump_outputs(path, inputs, outs, status, out_cap):
+    """Write what a caller of the timed path received in its last step, so that two builds can be compared output
+    for output on the same inputs:
+
+      status, out_len, out_crc32   per item: status code, encoded length, CRC-32 of the encoded file (float64)
+      input_crc32                  per item: CRC-32 of the input file, to confirm both runs saw the same inputs
+      sample_index, sample_bytes   the encoded files of the items dump_sample picks, their bytes as float32,
+                                   concatenated in sample_index order (split them with out_len[sample_index])"""
+    import zlib
+    os.makedirs(path, exist_ok=True)
+    pick = dump_sample(len(outs), out_cap)
+    arrays = {"status": np.asarray(status, np.float64),
+              "out_len": np.array([len(o) for o in outs], np.float64),
+              "out_crc32": np.array([zlib.crc32(o) for o in outs], np.float64),
+              "input_crc32": np.array([zlib.crc32(x) for x in inputs], np.float64),
+              "sample_index": pick.astype(np.float64),
+              "sample_bytes": np.frombuffer(b"".join(outs[i] for i in pick), np.uint8).astype(np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def dump_dir(args, rank, world):
+    return args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}")
 
 
 # ------------------------------------------------------------------------------ corpus
@@ -548,6 +595,9 @@ def main_x(args):
     sampler.end()
     clocks = sampler.stop()
     assert all(status[i] == 0 for i in range(n))
+    if args.dump_outputs:
+        dump_outputs(dump_dir(args, rank, world), [files[k] for k in idx],
+                     [C.string_at(out_ptrs[i], out_lens[i]) for i in range(n)], list(status), out_cap)
     kern_s = agg["ms_busy_max_lane"] / 1000.0
     kern_max, e2e_max = max_over_ranks([kern_s, e2e_s], dist, device="cuda")
     if rank == 0:
@@ -740,6 +790,8 @@ def main():
     outs, fst = b.fetch(n)
     assert all(s == 0 for s in fst), "device pipeline reported per-image failures"
     out_bytes = int(sum(len(o) for o in outs))
+    if args.dump_outputs:
+        dump_outputs(dump_dir(args, rank, world), [arena[o:o + l_] for o, l_ in zip(offs, lens)], outs, fst, out_cap)
 
     # ---------------- end to end: host buffers in, host buffers out, every step
     for _ in range(max(1, args.warmup // 2)):

@@ -1,7 +1,6 @@
 import os
 import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -15,7 +14,8 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    return np.load(os.path.join(ROOT, "tests", "golden", "golden.npz"))
+    from tests.golden import load
+    return load("golden")
 
 
 @pytest.fixture(scope="session")

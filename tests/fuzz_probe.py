@@ -9,12 +9,13 @@ import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from lilliput_b200 import abi  # noqa: E402
+from tests import golden as golden_set  # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def corpus():
-    g = np.load(os.path.join(ROOT, "tests", "golden", "golden.npz"))
+    g = golden_set.load("golden")
     w = np.load(os.path.join(ROOT, "tests", "golden", "webp_golden.npz"))
     j = np.load(os.path.join(ROOT, "tests", "golden", "jpeg_multiscan_golden.npz"))
     a = np.load(os.path.join(ROOT, "tests", "golden", "png_adam7_golden.npz"))

@@ -15,6 +15,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 from lilliput_b200 import abi  # noqa: E402
 from lilliput_b200.synth import synth_image  # noqa: E402
+from tests import golden as golden_set  # noqa: E402
 
 RESIZE_CASES = [  # (seed, src_w, src_h, ch, crop(x,y,w,h) or None, dst_w, dst_h, interpolation)
     (11, 1920, 1080, 3, (420, 0, 1080, 1080), 256, 256, 3),   # BASELINE config 2 geometry
@@ -187,8 +188,8 @@ def main():
         out[f"gifsha_{name}"] = np.array([hashlib.sha256(f.tobytes()).hexdigest() for f in frames])
         if frames.nbytes <= 200000:
             out[f"gifframes_{name}"] = frames
-    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "golden.npz"), **out)
-    print("wrote", len(out), "arrays,", os.path.getsize(os.path.join(ROOT, "tests/golden/golden.npz")), "bytes")
+    golden_set.save("golden", out)
+    print("wrote", len(out), "arrays")
 
 
 if __name__ == "__main__":

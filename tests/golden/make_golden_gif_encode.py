@@ -14,6 +14,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from lilliput_b200 import abi  # noqa: E402
+from tests import golden as golden_set  # noqa: E402
 
 TIMEOUT_NS = 600 * 10**9  # ops.go:368,435: a zero EncodeTimeout times out after the first frame
 
@@ -39,7 +40,7 @@ CASES = [  # (fixture, label, options)
 
 def main():
     ref = abi.load_reference()
-    g = np.load(os.path.join(ROOT, "tests", "golden", "golden.npz"))
+    g = golden_set.load("golden")
     out, names = {}, []
     for fixture, label, kw in CASES:
         data = g[f"gif_{fixture}"].tobytes()

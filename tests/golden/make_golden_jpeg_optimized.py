@@ -21,6 +21,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 from lilliput_b200 import abi  # noqa: E402
 from lilliput_b200.synth import synth_image  # noqa: E402
+from tests import golden as golden_set  # noqa: E402
 
 
 def cases():
@@ -74,9 +75,8 @@ def main():
             out[f"px_{name}"] = px
         print(f"{name:32s} {len(data):7d} B -> {px.shape}")
     out["names"] = np.array(names)
-    path = os.path.join(ROOT, "tests", "golden", "jpeg_optimized_golden.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path))
+    golden_set.save("jpeg_optimized_golden", out)
+    print("wrote", len(out), "arrays")
 
 
 if __name__ == "__main__":

@@ -22,14 +22,16 @@ g++ -O1 -g -std=c++17 -fsanitize=address,undefined -fno-omit-frame-pointer -I$RO
     -I${CUDA_HOME:-/usr/local/cuda}/include \
     $ROOT/tests/native/host_parse_fuzz.cpp -o $OUT/host_parse_fuzz -L$OUT -llp_asan -Wl,-rpath,$OUT
 python - <<PY
-import numpy as np, os
+import numpy as np, os, sys
 root, out = "$ROOT", "$OUT/seeds"
+sys.path.insert(0, root)
+from tests.golden import load  # merges the parts of a set stored as <name>.npz, <name>_2.npz, ...
 n = 0
-for f, prefixes in [("golden.npz", ("gif_", "png_", "jpeg_", "jpegvar_", "c1_input", "c6_input")),
-                    ("webp_golden.npz", ("webp_",)), ("jpeg_multiscan_golden.npz", ("jpg_",)),
-                    ("png_adam7_golden.npz", ("png_",)), ("jpeg_optimized_golden.npz", ("jpg_",)),
-                    ("gif_encode_golden.npz", ("out_",))]:
-    g = np.load(os.path.join(root, "tests", "golden", f))
+for f, prefixes in [("golden", ("gif_", "png_", "jpeg_", "jpegvar_", "c1_input", "c6_input")),
+                    ("webp_golden", ("webp_",)), ("jpeg_multiscan_golden", ("jpg_",)),
+                    ("png_adam7_golden", ("png_",)), ("jpeg_optimized_golden", ("jpg_",)),
+                    ("gif_encode_golden", ("out_",))]:
+    g = load(f)
     for k in g.files:
         a = g[k]
         if k.startswith(prefixes) and a.dtype == np.uint8 and a.ndim == 1 and 16 <= a.size <= 60000:

@@ -1,6 +1,6 @@
 """CPU: bench.py's clock sampler.  A timed region of the bench is a few hundred ms, so the sampler runs from
 before the warm-up and keeps only the samples stamped inside the timed windows; these tests pin that windowing,
-the throttle-reason decoding, and the nvidia-smi child path (a stand-in `nvidia-smi` script on PATH)."""
+the throttle-reason decoding, and the nvidia-smi child path (a stand-in `nvidia-smi` script on PATH, NVML kept out)."""
 import os
 import stat
 import sys
@@ -58,6 +58,10 @@ def test_nvidia_smi_child_path(tmp_path, monkeypatch):
     fake.chmod(fake.stat().st_mode | stat.S_IEXEC)
     monkeypatch.setenv("PATH", f"{tmp_path}:{os.environ['PATH']}")
     c = _sampler()
+
+    def no_nvml():
+        raise RuntimeError("NVML unavailable")
+    monkeypatch.setattr(c, "_nvml_open", no_nvml)   # where a GPU is, NVML would win over the child this test is about
     c.start()
     time.sleep(0.15)                    # "warm-up"
     c.begin()

@@ -11,6 +11,8 @@ import subprocess
 import numpy as np
 import pytest
 
+from tests import golden as golden_set
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OBJ = sorted(glob.glob(os.path.join(ROOT, "lilliput_b200", "csrc", "build", "*.o")))
 CUDA_INC = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "include")
@@ -36,7 +38,7 @@ def fake(tmp_path_factory):
                      ("host_transform_fuzz.cpp", "transform_fake")]:
         run(["g++", "-O1", "-g", "-std=c++17", *san, *inc, os.path.join(nat, src), "-o", exe, "-L.", "-llp_fake",
              "-Wl,-rpath," + d])
-    g = np.load(os.path.join(ROOT, "tests", "golden", "golden.npz"))
+    g = golden_set.load("golden")
     w = np.load(os.path.join(ROOT, "tests", "golden", "webp_golden.npz"))
     seeds = []
     for k, a in [("c1_input", g["c1_input"]), ("jpeg_31", g["jpeg_31"]), ("jpegvar_420_0", g["jpegvar_420_0"]),

@@ -4,15 +4,14 @@ reference itself decoded (tests/golden/jpeg_optimized_golden.npz).  Bit-exact.  
 what the Annex K tables never do: codes of every length, long codes behind several prefixes, tables
 with two or three symbols."""
 import hashlib
-import os
 
 import numpy as np
 import pytest
 
 from lilliput_b200 import abi
+from tests import golden as golden_set
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-G = np.load(os.path.join(ROOT, "tests", "golden", "jpeg_optimized_golden.npz"))
+G = golden_set.load("jpeg_optimized_golden")
 NAMES = [str(n) for n in G["names"]]
 
 
